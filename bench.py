@@ -2,6 +2,7 @@
 """bench.py — exposure-path traversals/sec on a synthetic estate (BASELINE.json's metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload L|M2|M1|S] [--mode exposure|enumerate] [--impl b200|reference]
+                    [--dump-outputs DIR]
 
 One *traversal* = for one finding node f: ``impact_of(f, max_depth=4)`` + f's derived exposure paths (SURVEY.md §8d).
 ``--mode enumerate`` (BASELINE config 5) adds, per finding, ``bfs(f, max_depth=4, traversable_only=True)`` path
@@ -324,6 +325,66 @@ def parity_gate(dg, og, est, host, my_host, args, mode: str) -> str:
     return msg
 
 
+# ── --dump-outputs ──────────────────────────────────────────────────────────────────────────────────────────────────────
+# The results of one step at L run to gigabytes, so a seeded sample of the findings is written: for each sampled finding its
+# complete per-query answers and the first entries of its node / edge lists and exposure-path rows (all layout-independent:
+# arena offsets are not written).  Everything is float64, which holds every int32 id exactly.
+DUMP_BYTES = 64 << 20             # all files together
+DUMP_QUERIES = 2048               # sampled findings
+DUMP_ROWS = 64                    # exposure-path rows kept per sampled finding
+DUMP_LIST_VALUES = 6 << 20        # list entries kept over all sampled findings and all walks of the step
+
+
+def _capped_index(start, count, cap: int):
+    """Positions start[i] .. start[i] + min(count[i], cap) - 1, concatenated over i."""
+    import torch
+
+    pos = torch.arange(cap, device=start.device)
+    keep = pos[None, :] < count[:, None]
+    return (start[:, None] + pos[None, :])[keep]
+
+
+def dump_outputs(out_dir: Path, roots, sel, walks, paths) -> None:
+    """Write what the device buffers of `walks` ((name, DeviceWalk) pairs) and `paths` (DevicePaths) hold for the queries `sel`
+    of the batch `roots` as `out_dir/<name>.npy`."""
+    import torch
+
+    from agent_bom_b200.graph.schema import N_ENTITY_TYPES
+
+    dev = roots.device
+    q = torch.from_numpy(sel).to(dev)
+    n_lists = sum(1 + (w.parent is not None) + (w.depth is not None) + (w.edges is not None) for _, w in walks)
+    cap = min(1024, DUMP_LIST_VALUES // (len(sel) * n_lists))
+    out = {"sources": roots[q]}
+    for name, w in walks:
+        p = name.replace("[", "_").rstrip("]")
+        count = w.q_count[q].long()
+        out[f"{p}_count"], out[f"{p}_maxd"], out[f"{p}_flags"] = count, w.q_maxd[q], w.q_flags[q]
+        if w.q_hist is not None:
+            out[f"{p}_hist"] = w.q_hist.view(-1, N_ENTITY_TYPES)[q]
+        ix = _capped_index(w.q_start[q], count, cap)
+        for field in ("nodes", "parent", "depth"):
+            if getattr(w, field) is not None:
+                out[f"{p}_{field}"] = getattr(w, field)[ix]
+        if w.edges is not None:
+            out[f"{p}_ecount"] = w.q_ecount[q]
+            out[f"{p}_edges"] = w.edges[_capped_index(w.q_estart[q], w.q_ecount[q], cap)]
+    first = paths.f_off[q]
+    rows = paths.f_off[q + 1] - first
+    ix = _capped_index(first, rows, DUMP_ROWS)
+    out["paths_count"], out["paths_hops"], out["paths_rels"] = rows, paths.hops.view(-1, 4)[ix], paths.rels.view(-1, 4)[ix, :3]
+    out["paths_ncred"], out["paths_ntool"] = paths.ncred[ix], paths.ntool[ix]
+    arrays = {k: v.cpu().numpy().astype(np.float64) for k, v in out.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_BYTES:
+        raise SystemExit(f"[bench] --dump-outputs: {total:,} bytes exceed the {DUMP_BYTES:,}-byte bound")
+    out_dir.mkdir(parents=True, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(out_dir / f"{k}.npy", a)
+    log(f"[bench] outputs of the last timed step: {len(sel):,} of {roots.shape[0]:,} findings, lists cut at {cap} entries and "
+        f"{DUMP_ROWS} path rows, {len(arrays)} arrays ({total / 1e6:.1f} MB) -> {out_dir}")
+
+
 def main() -> int:
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -339,7 +400,14 @@ def main() -> int:
     ap.add_argument("--check", type=int, default=2000, help="evenly spaced findings checked against the oracle before timing")
     ap.add_argument("--check-heavy", type=int, default=200, help="heaviest findings (by forecast degree) added to the parity gate")
     ap.add_argument("--no-overlap", dest="overlap", action="store_false", help="run the exposure-path pipeline after the walk instead of next to it (second stream)")
+    ap.add_argument("--dump-outputs", type=Path, metavar="DIR",
+                    help=f"after the timed steps write what the last one computed for a seeded sample of {DUMP_QUERIES} findings as DIR/<name>.npy "
+                         "(float64; rank 0's shard with several GPUs; the step must be one batch)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 path")
     if args.warmup < 3:
         args.warmup = 3
     claim_stdout()
@@ -390,6 +458,8 @@ def main() -> int:
     nq = int(my.shape[0])
     batch = max(1, min(args.batch, nq))
     batches = [(s, min(s + batch, nq)) for s in range(0, nq, batch)]
+    if args.dump_outputs and len(batches) > 1:
+        raise SystemExit(f"[bench] --dump-outputs needs the step in one batch: --batch {batch:,} < {nq:,} findings (the buffers keep only the last batch)")
     log(f"[bench] rank {info.rank}/{info.world}: {nq:,} findings in {len(batches)} batches of <= {batch:,}; CSR replicate {t_bcast:.3f}s ({dg.nbytes / 1e9:.2f} GB, {bstats})")
 
     # ---- cold first call through the host API (no size hint yet): arenas are sized on the fly, the walk may run twice
@@ -483,6 +553,9 @@ def main() -> int:
         one_step(overlap=args.overlap)
     end.record()
     torch.cuda.synchronize()
+    if args.dump_outputs and info.rank == 0:
+        sel = np.sort(np.random.default_rng(args.seed).choice(nq, size=min(DUMP_QUERIES, nq), replace=False))
+        dump_outputs(args.dump_outputs, my, sel, [("impact", walk), *extra], paths)
     abdist.barrier(info)
     launches = lib.abb_launch_count() - launches0
     dev_ms = start.elapsed_time(end)

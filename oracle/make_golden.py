@@ -26,6 +26,7 @@ from __future__ import annotations
 import gzip
 import importlib.util
 import json
+import lzma
 import random
 import sys
 from pathlib import Path
@@ -206,6 +207,16 @@ def graph_arrays(g: UnifiedGraph, ix: Indexer):
 
 
 def run_battery(name: str, g: UnifiedGraph, rng: random.Random, small: bool, derived: bool = True):
+    doc = battery_doc(name, g, rng, small, derived)
+    OUT.mkdir(parents=True, exist_ok=True)
+    path = OUT / f"{name}.json.gz"
+    with gzip.GzipFile(path, "wb", mtime=0) as fh:
+        fh.write(json.dumps(doc, separators=(",", ":"), sort_keys=True).encode())
+    print(f"{name}: {doc['n_real']} nodes (+{len(doc['node_ids']) - doc['n_real']} ghosts) {len(doc['edges'])} edges, "
+          f"{len(doc['findings'])} findings -> {path.name} {path.stat().st_size / 1024:.0f} KiB")
+
+
+def battery_doc(name: str, g: UnifiedGraph, rng: random.Random, small: bool, derived: bool = True) -> dict:
     ix = Indexer(g)
     node_types, edges, adj, radj = graph_arrays(g, ix)
     ids = ix.ids
@@ -328,11 +339,7 @@ def run_battery(name: str, g: UnifiedGraph, rng: random.Random, small: bool, der
         "agents": [ix(a) for a in agents],
         "cases": cases,
     }
-    OUT.mkdir(parents=True, exist_ok=True)
-    path = OUT / f"{name}.json.gz"
-    with gzip.GzipFile(path, "wb", mtime=0) as fh:
-        fh.write(json.dumps(doc, separators=(",", ":"), sort_keys=True).encode())
-    print(f"{name}: {ix.n_real} nodes (+{len(ids) - ix.n_real} ghosts) {len(edges)} edges, {len(findings)} findings -> {path.name} {path.stat().st_size / 1024:.0f} KiB")
+    return doc
 
 
 def estate_identity():
@@ -980,7 +987,83 @@ def envelope_golden():
         fh.write(json.dumps({"cases": cases}, sort_keys=True).encode())
 
 
+# ── random estates (tests/test_oracle_vs_reference_live.py) ─────────────────────────────────────────────────────────────
+LIVE_SEEDS = list(range(11, 27))
+
+
+def random_estate(seed: int) -> UnifiedGraph:
+    """A typed multigraph through the reference's own add_node / add_edge: an estate-shaped core (agents → servers → packages →
+    vulnerabilities, credentials, tools) plus noise edges of every relationship type, bidirectional and non-traversable edges,
+    duplicates, self loops and ghost endpoints."""
+    rng = random.Random(seed)
+    ET = EntityType
+    n_agents, n_servers, n_pkgs = rng.randint(2, 6), rng.randint(3, 9), rng.randint(4, 12)
+    n_vulns, n_creds, n_tools = rng.randint(3, 14), rng.randint(1, 6), rng.randint(1, 6)
+    sev = ["", "low", "medium", "high", "critical"]
+    nodes, edges = [], []
+
+    def add(prefix, count, et, with_risk=False):
+        ids = []
+        for i in range(count):
+            nid = f"{prefix}:{seed}:{rng.randrange(10**6):06d}:{i}"
+            ids.append(nid)
+            if with_risk:
+                nodes.append((nid, et, rng.choice(sev), rng.choice([0.0, 0.0, 3.5, 7.5, 9.8]), f"{prefix.upper()}-{i}"))
+            else:
+                nodes.append((nid, et))
+        return ids
+
+    agents, servers, pkgs = add("agent", n_agents, ET.AGENT), add("server", n_servers, ET.SERVER), add("pkg", n_pkgs, ET.PACKAGE)
+    vulns = add("vuln", n_vulns, ET.VULNERABILITY, True) + add("mis", rng.randint(0, 3), ET.MISCONFIGURATION, True)
+    creds, tools = add("cred", n_creds, ET.CREDENTIAL), add("tool", n_tools, ET.TOOL)
+    extra = add("user", rng.randint(0, 2), ET.USER) + add("model", rng.randint(0, 2), ET.MODEL) + add("prov", rng.randint(0, 1), ET.PROVIDER)
+    rng.shuffle(nodes)                       # insertion order is what discovery order hangs on
+    for a in agents:
+        for s in rng.sample(servers, rng.randint(1, min(3, len(servers)))):
+            edges.append((a, s, R.USES))
+    for s in servers:
+        for p in rng.sample(pkgs, rng.randint(0, min(4, len(pkgs)))):
+            edges.append((s, p, R.DEPENDS_ON))
+        for c in rng.sample(creds, rng.randint(0, min(3, len(creds)))):
+            edges.append((s, c, R.EXPOSES_CRED))
+        for t in rng.sample(tools, rng.randint(0, min(3, len(tools)))):
+            edges.append((s, t, R.PROVIDES_TOOL))
+        if rng.random() < 0.3:
+            edges.append((s, rng.choice(vulns), R.VULNERABLE_TO))
+    for p in pkgs:
+        for v in rng.sample(vulns, rng.randint(0, min(3, len(vulns)))):
+            edges.append((p, v, R.VULNERABLE_TO))
+        if rng.random() < 0.3:
+            edges.append((p, rng.choice(pkgs), R.DEPENDS_ON))          # transitive dependency (possibly a self loop)
+    for v in rng.sample(vulns, min(3, len(vulns))):
+        edges.append((v, rng.choice(pkgs), R.AFFECTS))
+    everything = agents + servers + pkgs + vulns + creds + tools + extra
+    rels = list(R)
+    for _ in range(rng.randint(8, 30)):                                  # noise: any relationship, direction, traversability
+        a, b = rng.choice(everything), rng.choice(everything)
+        edges.append((a, b, rng.choice(rels), rng.choice(["directed", "directed", "bidirectional"]), rng.random() > 0.2))
+    for _ in range(rng.randint(0, 3)):                                   # ghost endpoints
+        edges.append((rng.choice(everything), f"ghost:{seed}:{rng.randrange(1000)}", rng.choice(rels)))
+        edges.append((f"ghost:{seed}:{rng.randrange(1000)}", rng.choice(everything), rng.choice(rels)))
+    edges += rng.sample(edges, min(5, len(edges)))                       # exact duplicates: add_edge keeps the first
+    rng.shuffle(edges)
+    return mk(nodes, edges)
+
+
+def live_golden():
+    """tests/golden/live/estates.json.xz: the list of small-battery fixtures, one random estate per seed, in one xz stream
+    (per-file gzip would be half as large again)."""
+    docs = [battery_doc(f"live_{seed}", random_estate(seed), random.Random(seed), small=True) for seed in LIVE_SEEDS]
+    path = OUT / "live" / "estates.json.xz"
+    path.parent.mkdir(parents=True, exist_ok=True)
+    path.write_bytes(lzma.compress(json.dumps(docs, separators=(",", ":"), sort_keys=True).encode(), preset=9 | lzma.PRESET_EXTREME))
+    print(f"live estates: {len(docs)} seeds -> {path.name} {path.stat().st_size / 1024:.0f} KiB")
+
+
 def main():
+    if "--live-only" in sys.argv:
+        live_golden()
+        return
     if "--envelope-only" in sys.argv:
         envelope_golden()
         return
@@ -1012,6 +1095,7 @@ def main():
     effective_reach_golden()
     centrality_golden()
     lateral_golden()
+    live_golden()
     rng = random.Random(20260921)
     run_battery("kat_schema", kat_schema(), rng, small=True)
     run_battery("kat_directed", kat_directed(), rng, small=True)

@@ -1,109 +1,40 @@
-"""Live differential check of the CPU oracle against the UNMODIFIED reference engine on freshly generated random estates.
+"""Differential check of the CPU oracle against the UNMODIFIED reference engine on random estates.
 
-The committed fixtures (tests/golden/, made by oracle/make_golden.py) pin the oracle on fixed graphs; this test makes NEW graphs on
-every seed listed below — an estate-shaped core (agents → servers → packages → vulnerabilities, credentials, tools) plus noise
-edges of every relationship type, bidirectional and non-traversable edges, duplicates, self loops and ghost endpoints — runs the
-reference's own `impact_of / bfs / reachable_from / shortest_path / traverse_subgraph / compute_dependency_reach /
-_derived_attack_paths` on them (make_golden.run_battery) and holds the oracle to the same answers through the checks of
-tests/test_oracle_golden.py.
-
-Needs the reference tree (``/root/reference/src``), which exists in the build container only: skipped elsewhere (the GPU box has no
-reference; nothing under ``-m gpu`` depends on this file)."""
+The other fixtures under tests/golden/ pin the oracle on fixed known-answer graphs and generator estates; this test adds one
+random graph per seed (oracle/make_golden.py ``random_estate``) — an estate-shaped core (agents → servers → packages →
+vulnerabilities, credentials, tools) plus noise edges of every relationship type, bidirectional and non-traversable edges,
+duplicates, self loops and ghost endpoints — with the reference's own `impact_of / bfs / reachable_from / shortest_path /
+traverse_subgraph / compute_dependency_reach / _derived_attack_paths` answers on each (``make_golden.py --live-only`` runs the
+reference and writes them to ``tests/golden/live/estates.json.xz``), and holds the oracle to the same answers through the checks
+of tests/test_oracle_golden.py.  CPU-only."""
 
 from __future__ import annotations
 
-import random
-import sys
-from pathlib import Path
+import gzip
+import json
+import lzma
 
 import pytest
 
-REF_SRC = Path("/root/reference/src")
-pytestmark = pytest.mark.skipif(not (REF_SRC / "agent_bom" / "graph").exists(), reason="reference tree not present (build container only)")
+import golden_util
 
-ROOT = Path(__file__).resolve().parents[1]
-SEEDS = list(range(11, 27))
-
-
-def random_estate(mg, seed: int):
-    """A typed multigraph through the reference's own add_node / add_edge (make_golden.mk)."""
-    rng = random.Random(seed)
-    ET, R = mg.EntityType, mg.RelationshipType
-    n_agents, n_servers, n_pkgs = rng.randint(2, 6), rng.randint(3, 9), rng.randint(4, 12)
-    n_vulns, n_creds, n_tools = rng.randint(3, 14), rng.randint(1, 6), rng.randint(1, 6)
-    sev = ["", "low", "medium", "high", "critical"]
-    nodes, edges = [], []
-
-    def add(prefix, count, et, with_risk=False):
-        ids = []
-        for i in range(count):
-            nid = f"{prefix}:{seed}:{rng.randrange(10**6):06d}:{i}"
-            ids.append(nid)
-            if with_risk:
-                nodes.append((nid, et, rng.choice(sev), rng.choice([0.0, 0.0, 3.5, 7.5, 9.8]), f"{prefix.upper()}-{i}"))
-            else:
-                nodes.append((nid, et))
-        return ids
-
-    agents, servers, pkgs = add("agent", n_agents, ET.AGENT), add("server", n_servers, ET.SERVER), add("pkg", n_pkgs, ET.PACKAGE)
-    vulns = add("vuln", n_vulns, ET.VULNERABILITY, True) + add("mis", rng.randint(0, 3), ET.MISCONFIGURATION, True)
-    creds, tools = add("cred", n_creds, ET.CREDENTIAL), add("tool", n_tools, ET.TOOL)
-    extra = add("user", rng.randint(0, 2), ET.USER) + add("model", rng.randint(0, 2), ET.MODEL) + add("prov", rng.randint(0, 1), ET.PROVIDER)
-    rng.shuffle(nodes)                       # insertion order is what discovery order hangs on
-    for a in agents:
-        for s in rng.sample(servers, rng.randint(1, min(3, len(servers)))):
-            edges.append((a, s, R.USES))
-    for s in servers:
-        for p in rng.sample(pkgs, rng.randint(0, min(4, len(pkgs)))):
-            edges.append((s, p, R.DEPENDS_ON))
-        for c in rng.sample(creds, rng.randint(0, min(3, len(creds)))):
-            edges.append((s, c, R.EXPOSES_CRED))
-        for t in rng.sample(tools, rng.randint(0, min(3, len(tools)))):
-            edges.append((s, t, R.PROVIDES_TOOL))
-        if rng.random() < 0.3:
-            edges.append((s, rng.choice(vulns), R.VULNERABLE_TO))
-    for p in pkgs:
-        for v in rng.sample(vulns, rng.randint(0, min(3, len(vulns)))):
-            edges.append((p, v, R.VULNERABLE_TO))
-        if rng.random() < 0.3:
-            edges.append((p, rng.choice(pkgs), R.DEPENDS_ON))          # transitive dependency (possibly a self loop)
-    for v in rng.sample(vulns, min(3, len(vulns))):
-        edges.append((v, rng.choice(pkgs), R.AFFECTS))
-    everything = agents + servers + pkgs + vulns + creds + tools + extra
-    rels = list(R)
-    for _ in range(rng.randint(8, 30)):                                  # noise: any relationship, direction, traversability
-        a, b = rng.choice(everything), rng.choice(everything)
-        edges.append((a, b, rng.choice(rels), rng.choice(["directed", "directed", "bidirectional"]), rng.random() > 0.2))
-    for _ in range(rng.randint(0, 3)):                                   # ghost endpoints
-        edges.append((rng.choice(everything), f"ghost:{seed}:{rng.randrange(1000)}", rng.choice(rels)))
-        edges.append((f"ghost:{seed}:{rng.randrange(1000)}", rng.choice(everything), rng.choice(rels)))
-    edges += rng.sample(edges, min(5, len(edges)))                       # exact duplicates: add_edge keeps the first
-    rng.shuffle(edges)
-    return mg.mk(nodes, edges)
+BUNDLE = golden_util.GOLDEN / "live" / "estates.json.xz"
 
 
 @pytest.fixture(scope="module")
 def live(tmp_path_factory):
-    import importlib.util
-
-    import golden_util
-
-    spec = importlib.util.spec_from_file_location("abb_make_golden", ROOT / "oracle" / "make_golden.py")
-    mg = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mg)          # puts the reference's src on sys.path and imports agent_bom.graph
-
+    """Unpack the bundle into one fixture file per seed, where golden_util.load looks for them."""
+    docs = json.loads(lzma.decompress(BUNDLE.read_bytes()))
     out = tmp_path_factory.mktemp("live_golden")
-    saved = (mg.OUT, golden_util.GOLDEN)
-    mg.OUT = golden_util.GOLDEN = out
+    for doc in docs:
+        with gzip.open(out / f"{doc['name']}.json.gz", "wb") as fh:
+            fh.write(json.dumps(doc).encode())
+    saved = golden_util.GOLDEN
+    golden_util.GOLDEN = out
     try:
-        names = []
-        for seed in SEEDS:
-            name = f"live_{seed}"
-            mg.run_battery(name, random_estate(mg, seed), random.Random(seed), small=True)
-            names.append(name)
-        yield names
+        yield [doc["name"] for doc in docs]
     finally:
-        mg.OUT, golden_util.GOLDEN = saved
+        golden_util.GOLDEN = saved
 
 
 @pytest.mark.parametrize("check", ["test_adjacency_model", "test_impact_of", "test_bfs_paths_exact_order", "test_reachable_from", "test_shortest_path",
@@ -112,5 +43,6 @@ def test_oracle_equals_the_reference_on_fresh_random_estates(live, check):
     import test_oracle_golden as tog
 
     fn = getattr(tog, check)
+    assert len(live) == 16
     for name in live:
         fn(name)
